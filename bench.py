@@ -118,8 +118,16 @@ def parse():
                          "the same second, i.e. what an owner behind that many senders receives")
     ap.add_argument("--shuffle", default="partials", choices=["partials", "rows"],
                     help="N>1: what crosses the all-to-all (per-pane partial aggregates, or raw rows)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the windows the last timed step emitted under DIR as float64 "
+                         ".npy files, exactly (avg.npy; <column>_hi.npy / <column>_lo.npy = upper / lower 32 bits of "
+                         "every int64 column), rows ordered by window and key, a seeded row sample above 64 MB: the "
+                         "sliding workload at N = 1")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.workload != "sliding" or args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs writes the device-resident sliding-window path of one GPU: "
+                 "--workload sliding --impl ours at N = 1")
     args.native_exchange = (not args.python_exchange) and (world <= 4 or args.native_exchange)
     return args
 
@@ -411,6 +419,46 @@ def window_checksums(torch, device, emitted):
     return out
 
 
+OUT_COLS = ("key", "window_start", "window_end", "sum", "avg", "count", "_timestamp")  # handle_watermark_device's order
+DUMP_BYTES = 64_000_000
+
+
+def window_columns(torch, device, emitted):
+    """Host copies of the windows of one emission left on the device (`emitted` as in window_checksums), one int64
+    array per OUT_COLS name (avg: float64), rows ordered by (window start, key): the order the operator emits rows in
+    follows its dictionary layout, which is not part of the result."""
+    import numpy as np
+
+    from arroyo_b200.multi_gpu import _Ptr
+    parts = [[torch.as_tensor(_Ptr(cols[c], n), device=device).cpu().numpy() for c in range(len(OUT_COLS))]
+             for n, cols in emitted if n]
+    cols = [np.concatenate(c) for c in zip(*parts)]
+    order = np.lexsort((cols[0], cols[1]))
+    out = {name: c[order] for name, c in zip(OUT_COLS, cols)}
+    out["avg"] = out["avg"].view(np.float64)
+    return out
+
+
+def dump_outputs(out_dir, cols):
+    """Writes the columns as float64 .npy files under out_dir, every value exactly: a float64 column as <name>.npy, an
+    int64 column (keys and nanosecond timestamps need more than float64's 53 bits) as <name>_hi.npy, its upper 32 bits
+    (signed), and <name>_lo.npy, its lower 32 bits (unsigned): value = hi * 2^32 + lo.  Above DUMP_BYTES in all, every
+    file keeps the same fixed, seeded sample of rows."""
+    import numpy as np
+    files = {}
+    for name, c in cols.items():
+        if c.dtype == np.float64:
+            files[name] = c
+        else:
+            files[name + "_hi"], files[name + "_lo"] = c >> 32, c & 0xFFFFFFFF
+    n = len(cols["key"])
+    cap = (DUMP_BYTES - 1024 * len(files)) // (8 * len(files))  # 1 KB per file for its .npy header
+    rows = np.sort(np.random.default_rng(0).choice(n, cap, replace=False)) if n > cap else slice(None)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, c in files.items():
+        np.save(os.path.join(out_dir, name + ".npy"), c[rows].astype(np.float64))
+
+
 def compare_windows(got, want, min_windows):
     """got: {wstart: (wend, rows_out, counts, sums, avgs)} from the GPU run; want: the oracle's window list.
     Bit-exact rows / counts / sums (wrapping), AVG checksum within 1e-6 relative (north-star tolerance)."""
@@ -492,10 +540,12 @@ def bind_to_gpu_numa_node(local):
         return f"unchanged ({type(e).__name__}: {e})"
 
 
-def device_resident(args, torch, native, ffi, local, panes, W, K, rows, collect=False, sampler=None):
+def device_resident(args, torch, native, ffi, local, panes, W, K, rows, collect=False, sampler=None, last_window=None):
     """W warm-up + K timed steps over `panes` (already in HBM); CUDA events on the operator's stream.
     Returns (ms, stats delta, rows emitted, clocks, per-window checksums if `collect`).  With `collect` every emitted
-    window is reduced to checksums on the device (torch kernels inside the loop): that pass verifies, it is not timed."""
+    window is reduced to checksums on the device (torch kernels inside the loop): that pass verifies, it is not timed.
+    A dict passed as `last_window` receives the host columns of the emission the last timed step began
+    (window_columns), copied after the timed region; it is an error if that step began none, or more than one."""
     import pyarrow as pa
     device = torch.device("cuda", local)
     plans = build_batch_lists(torch, panes, rows)
@@ -507,16 +557,19 @@ def device_resident(args, torch, native, ffi, local, panes, W, K, rows, collect=
                                              flags=flags, expected_keys=args.keys, chunk_log2=args.chunk_log2)
     rows_out = 0
     sums = {}
+    last_step, last, n_last = W + K - 1, [], 0  # the last timed step's emission and how many it began
 
-    outstanding = False
+    outstanding = None  # the step that began the emission still to be polled
 
     def gather():
         # the windows of the outstanding emission (arroyo_b200_op_handle_watermark_device_poll)
-        nonlocal rows_out, outstanding
-        if not outstanding:
+        nonlocal rows_out, outstanding, last, n_last
+        if outstanding is None:
             return
-        outstanding = False
+        by, outstanding = outstanding, None
         emitted = op.handle_watermark_device_poll()
+        if by == last_step:
+            last, n_last = emitted, n_last + 1
         for n, _ in emitted:
             rows_out += n
         if collect:
@@ -533,14 +586,14 @@ def device_resident(args, torch, native, ffi, local, panes, W, K, rows, collect=
             if wm is None:
                 continue
             if args.sync_emit:
-                outstanding = True
+                outstanding = p
                 op.handle_watermark_device_begin(wm)
                 gather()
                 continue
             op.submit()
             gather()
             op.handle_watermark_device_begin(wm)
-            outstanding = True
+            outstanding = p
 
     if sampler is None:
         sampler = ClockSampler(local)
@@ -565,6 +618,13 @@ def device_resident(args, torch, native, ffi, local, panes, W, K, rows, collect=
     sampler.end()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if not collect else None
+    if last_window is not None:
+        # flush() emits nothing: the buffers still hold the last emission until the operator's next one (which is also
+        # why only one emission of the step can be read here)
+        if n_last != 1 or not any(n for n, _ in last):
+            raise RuntimeError(f"the last timed step began {n_last} emissions (rows: {[n for n, _ in last]}); "
+                               "--dump-outputs writes the windows of its one emission")
+        last_window.update(window_columns(torch, device, last))
     st1 = op.stats()
     op.close()
     del plans
@@ -610,8 +670,12 @@ def run_ours(args):
     assert rows % BATCH_ROWS == 0
     gen_pane = make_generator(torch, device, rows, args.keys, args.dist, 42 + rank, args.keyspace)
     panes = [gen_pane(p) for p in range(W + K)]
-    ms, d, rows_out, clocks, _ = device_resident(args, torch, native, ffi, local, panes, W, K, rows)
+    last_window = {} if args.dump_outputs else None
+    ms, d, rows_out, clocks, _ = device_resident(args, torch, native, ffi, local, panes, W, K, rows,
+                                                 last_window=last_window)
     del panes
+    if last_window is not None:
+        dump_outputs(args.dump_outputs, last_window)
 
     value = K * rows / (ms * 1e-3)
     peak, peak_kind = measured_peak()

@@ -469,7 +469,7 @@ def run(args, B):
         dist_mod.init_process_group("nccl", device_id=device)
         dist = dist_mod
     torch.cuda.set_stream(torch.cuda.Stream(device=device))
-    steps = min(args.steps, 20)
+    steps = args.steps
     sampler = B.ClockSampler(local) if rank == 0 else None
     if args.workload == "join":
         n_p, n_a, warm = 1 << args.join_persons_log2, 1 << args.join_auctions_log2, 3
