@@ -39,7 +39,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     ]
     if verbose:
         flags += ["-Xptxas", "-v"]
-    for knob in ("AB_INGEST_MIN_BLOCKS", "AB_INGEST_PREFETCH", "AB_P1_THREADS"):  # tuning knobs for experiments
+    for knob in ("AB_INGEST_MIN_BLOCKS", "AB_INGEST_PREFETCH", "AB_P1_THREADS", "AB_P1_RPT"):  # tuning knobs for experiments
         if os.environ.get(knob):
             flags += [f"-D{knob}=" + os.environ[knob]]
     build_dir = os.path.join(HERE, "build")

@@ -1908,6 +1908,15 @@ void WindowAggOp::launch_segments(const std::vector<Segment>& segs_in, int chunk
     tiles += (hs[i].n + TILE - 1) / TILE;
     rows += (uint64_t)hs[i].n;
   }
+  const bool two_pass = two_pass_eligible(rows);
+  long long t2 = 0;
+  if (two_pass) {
+    // tiles of the partition kernel are larger: the segment table is cut for them
+    for (size_t i = 0; i < segs_in.size(); ++i) {
+      hs[i].tile_start = t2;
+      t2 += (hs[i].n + P1_TILE - 1) / P1_TILE;
+    }
+  }
   AB_CUDA(cudaMemcpyAsync(d_segs_[li].p, hs, segs_in.size() * sizeof(Segment), cudaMemcpyHostToDevice, stream_));
   if (ring_ > RING_INLINE) upload_ring();
   if (!defer_[defer_cur_][0].p) {
@@ -1952,15 +1961,7 @@ void WindowAggOp::launch_segments(const std::vector<Segment>& segs_in, int chunk
   int grid = (int)std::min<long long>(tiles, (long long)num_sms_ * 8);
   if (grid < 1) grid = 1;
   if (profile_) AB_CUDA(cudaEventRecord(L.t0, stream_));
-  const bool two_pass = two_pass_eligible(rows);
   if (two_pass) {
-    // tiles of the partition kernel are larger: the segment table is re-cut for them
-    long long t2 = 0;
-    for (size_t i = 0; i < segs_in.size(); ++i) {
-      hs[i].tile_start = t2;
-      t2 += (hs[i].n + P1_TILE - 1) / P1_TILE;
-    }
-    AB_CUDA(cudaMemcpyAsync(d_segs_[li].p, hs, segs_in.size() * sizeof(Segment), cudaMemcpyHostToDevice, stream_));
     p.n_tiles = t2;
     launch_two_pass(p, rows, t2);
   }
